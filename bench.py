@@ -40,6 +40,7 @@ WORKLOADS = {
 }
 LAMBDA, ALPHA, SEED = 0.01, 1.0, 3
 PARITY_TOL = 1e-4
+DUMP_BYTES = 60_000_000      # --dump-outputs stays below 64 MB including the .npy headers
 
 
 def algorithmic_work(nu, ni, nnz, k, implicit):
@@ -194,18 +195,14 @@ def load_oracle():
         import ctypes
         import shutil
         if shutil.which("gcc"):
-            # -march=native code must not travel between machines: key the file by this host's CPU flags
-            import hashlib
-            flags = ""
-            try:
-                flags = next(ln for ln in open("/proc/cpuinfo") if ln.startswith("flags"))
-            except Exception:
-                pass
-            so = o._SO.parent / f"libals_oracle_native_{hashlib.sha1(flags.encode()).hexdigest()[:10]}.so"
-            if not so.exists() or so.stat().st_mtime < o._SRC.stat().st_mtime:
+            # -march=native code must not travel between machines, and the tree may be read-only: build it for this
+            # host in a temporary directory on every run (under a second); the loaded library outlives the directory
+            import tempfile
+            with tempfile.TemporaryDirectory(prefix="pio_oracle_") as tmp:
+                so = Path(tmp) / "libals_oracle_native.so"
                 subprocess.run(["gcc", "-O3", "-march=native", "-fopenmp", "-fPIC", "-shared", "-fvisibility=hidden",
                                 "-o", str(so), str(o._SRC), "-lm"], check=True)
-            o._lib = ctypes.CDLL(str(so))
+                o._lib = ctypes.CDLL(str(so))
             o._lib.oracle_num_threads.restype = ctypes.c_int
     except Exception:
         pass
@@ -305,6 +302,25 @@ def parity_sample(o, prob, src_u, new_i, new_u, n_user=2000, n_item=500, n_heavy
 def factor_checksum(uf, itf):
     """64-bit value: CRC32 of the user factor bytes (high word) and of the item factor bytes (low word)."""
     return f"{zlib.crc32(np.ascontiguousarray(uf).view(np.uint8)):08x}{zlib.crc32(np.ascontiguousarray(itf).view(np.uint8)):08x}"
+
+
+def dump_outputs(out_dir, uf, itf, uh, ih):
+    """--dump-outputs: what pio_als_get_factors hands a caller after the timed run (factors and has-flags of both sides)
+    as .npy files, so that two builds can be compared output for output.  Both sides keep the same fixed, seeded
+    fraction of their rows, chosen to stay under DUMP_BYTES; <side>_rows.npy holds the indices of the rows kept."""
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    row_bytes = 4 * uf.shape[1] + 4 + 8        # factor row (float32), has-flag (float32), row index (float64)
+    frac = min(1.0, DUMP_BYTES / (row_bytes * (uf.shape[0] + itf.shape[0])))
+    rng = np.random.default_rng(SEED)
+    for side, f, has in (("user", uf, uh), ("item", itf, ih)):
+        n = f.shape[0]
+        keep = int(n * frac)
+        rows = np.arange(n) if keep >= n else np.sort(rng.choice(n, keep, replace=False))
+        np.save(out_dir / f"{side}_factors.npy", np.ascontiguousarray(f[rows], np.float32))
+        np.save(out_dir / f"{side}_has.npy", has[rows].astype(np.float32))
+        np.save(out_dir / f"{side}_rows.npy", rows.astype(np.float64))
+    return {"dir": str(out_dir), "rows_fraction": frac}
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -459,7 +475,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-topk", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the factors of the timed run (a seeded sample of rows, < 64 MB) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
     nu, ni, nnz, k, implicit = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -549,6 +571,7 @@ def main():
     if rank == 0:
         uf_T, itf_T, uh, ih = m.get_factors()
     checksum = factor_checksum(uf_T, itf_T) if rank == 0 else None
+    dumped = dump_outputs(args.dump_outputs, uf_T, itf_T, uh, ih) if args.dump_outputs and rank == 0 else None
     if want_parity:
         m.run(1)
         if rank == 0:
@@ -690,6 +713,8 @@ def main():
            "roofline": roofline}
     if e2e:
         out["e2e"] = e2e
+    if dumped:
+        out["dumped_outputs"] = dumped
 
     rc = 0
     need_host = (want_parity or (not args.no_cpu_baseline and args.gpus == 1) or not args.no_topk)

@@ -1,6 +1,6 @@
 import os, sys, ctypes as C
 os.environ["PIO_ALS_TC_DEBUG"] = "1"
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 import pio_b200
 from pio_b200 import native, synth

@@ -4,7 +4,7 @@ then  PIO_ALS_TC=1 [PIO_ALS_TC_MIN_DEG=...] python tools/tc_timing.py   (TC_NU /
 The warp -> role map below matches the partition instantiated in pio_als.cu (2 gather, 5 converter warps, 2 teams)."""
 import os, sys, ctypes as C
 os.environ["PIO_ALS_TC_TIMING"] = "1"
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 import pio_b200
 from pio_b200 import native
