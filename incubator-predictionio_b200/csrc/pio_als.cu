@@ -1510,7 +1510,7 @@ static int create_common(pio_als_handle* h) {
     }
   }
   {
-    // Rank 33..64 kernel selection.  Default: the pair kernel (als_pair_kernel.cuh: mma.sync 3xTF32 Gramian, two rows per
+    // Rank 33..64 kernel selection.  Default: the pair kernel (als_pair_kernel.cuh: mma.sync split-FP16 Gramian, two rows per
     // warp, lockstep Cholesky) for every side -- measured at C2 it is the fastest on both sides (user half-step 18.7 ms,
     // item half-step 12.9 ms vs 17.1 ms for the tcgen05 kernel) and, with rows above 1024 ratings summed in two
     // levels, inside the parity bound on long rows.  PIO_ALS_TC=1: the tcgen05 Gramian kernel (als_tc_kernel.cuh) for
